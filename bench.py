@@ -39,6 +39,9 @@ random-weight OSNet (no pretrained file exists offline) and synthetic frames -- 
 per-frame cross-stream exchange (peer memory over NVLink, NCCL all-gather as the fallback) to the timed
 region; at N > 1 the default line measures it in its ``shared_gallery`` block.
 ``--impl reference`` times that CPU oracle alone and prints the same line.
+``--dump-outputs DIR`` saves what the timed loop returned for its last frame (track rows, and the detector
+post-process output) as .npy files; the inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 """
 from __future__ import annotations
 
@@ -478,14 +481,20 @@ def run_gpu_config(args, device, rank, world, lib, barrier, max_over_ranks, K, W
     l0 = lib.ssb_launch_count()
     e0.record(st)
     for k in range(K):
-        trk.update_pipelined(frame_dets(W + k, pstream), imgs_dev[W + k], lag=PIPE_LAG)
+        d_last = frame_dets(W + k, pstream)
+        trk.update_pipelined(d_last, imgs_dev[W + k], lag=PIPE_LAG)
         if gal is not None:
             gal.step()                     # export + exchange + cross-stream match, inside the timed region
-    trk.flush_pipelined()
+    rows_last = trk.flush_pipelined()
     if gal is not None:
         st.wait_stream(gal.stream)
     e1.record(st)
     barrier()
+    # what a caller of the timed path receives for the last timed frame (--dump-outputs); copied before the
+    # detector post-process slots are reused below
+    res["outputs"] = {"tracks": np.asarray(rows_last, dtype=np.float64)}
+    if use_post:
+        res["outputs"]["detections"] = d_last.cpu().numpy()
     launches = int(lib.ssb_launch_count() - l0)
     t_ms = max_over_ranks(e0.elapsed_time(e1))
     res["clocks"] = clocks.stop()
@@ -638,7 +647,13 @@ def main():
     ap.add_argument("--shared-gallery", action="store_true",
                     help="config C5's optional exchange: every stream's confirmed-track features exchanged after each "
                          "frame and matched across streams (read-only), inside the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed path returned for its last frame to DIR "
+                         "(rank 0): tracks.npy, float64 [M,7] rows x1,y1,x2,y2,track_id,class_id,conf; "
+                         "detections.npy, float32 [N,6] detector post-process output (C2 only)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; the reference arm has none")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -679,6 +694,10 @@ def main():
     K, W = args.steps, max(args.warmup, 3)
     want_cpu = rank == 0 and world == 1 and not args.no_cpu_baseline
     r = run_gpu_config(args, device, rank, world, lib, barrier, max_over_ranks, K, W, want_cpu)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in r["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
 
     reid_flops = 2.0 * REID_MACS_PER_CROP * r["reid_n"]
     achieved_tf = reid_flops / (r["reid_ms"] * 1e-3) / 1e12

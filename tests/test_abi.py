@@ -3,6 +3,8 @@
 import ctypes
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -103,10 +105,16 @@ def test_bn_fold_matches_unfolded_oracle(state_dict):
 
 
 def test_no_cpu_fallback():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from strongsort_yolo_b200 import _lib
-    from strongsort_yolo_b200.strong_sort import StrongSORT
-    with pytest.raises(_lib.SsbError):
-        StrongSORT()
+    """Without a CUDA device the tracker refuses to construct.  The devices are hidden from a child process, so
+    the check also runs on a machine that has a GPU."""
+    code = (f"import sys\nsys.path.insert(0, {ROOT!r})\n"
+            "from strongsort_yolo_b200 import _lib\n"
+            "from strongsort_yolo_b200.strong_sort import StrongSORT\n"
+            "try:\n"
+            "    StrongSORT()\n"
+            "except _lib.SsbError:\n"
+            "    raise SystemExit(0)\n"
+            "raise SystemExit('StrongSORT() constructed without a CUDA device')\n")
+    p = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=300)
+    assert p.returncode == 0, p.stdout[-2000:] + p.stderr[-2000:]
